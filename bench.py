@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the CPU restatement (reference arm)
     torchrun --nproc-per-node N ... bench.py --gpus N ...     # N > 1: one rank per GPU
+    python bench.py ... --dump-outputs DIR                     # + the last timed step's outputs as DIR/*.npy
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on that fits one GPU):
 10,000 pods x 4 GPUs x 1,800 samples (30 min @ 1 s) of synthetic DCGM_FI_DEV_GPU_UTIL per B200,
@@ -180,6 +181,8 @@ def run_reference(args):
         for i in range(args.steps):
             run(i, pods)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dbits[:(pods + 31) // 32], counts)
     dt = min(times)
     samples = pods * GPUS * SAMPLES
     value = samples * args.steps / dt
@@ -216,6 +219,16 @@ def step_stats(durations_us):
         return {"median_us": None, "p95_us": None, "min_us": None, "max_us": None}
     return {"median_us": float(np.median(d)), "p95_us": float(d[min(d.size - 1, int(np.ceil(0.95 * d.size)) - 1)]),
             "min_us": float(d[0]), "max_us": float(d[-1])}
+
+
+def dump_outputs(out_dir, decision_bits, counts):
+    """what a caller of the timed path receives from its last step, as float64 (exact for uint32 words):
+    decision_bits.npy = the packed per-pod idle bitmap (rank-major words at N > 1), counts.npy =
+    [n_series, n_candidates, n_decisions] summed over ranks"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "decision_bits.npy"), np.asarray(decision_bits, np.uint32).astype(np.float64))
+    np.save(os.path.join(out_dir, "counts.npy"), np.asarray(counts, np.float64))
 
 
 def run_cuda(args):
@@ -375,6 +388,8 @@ def run_cuda(args):
     last_bits = global_bits()
     last_counts = reduce_sum_i((int(ress[n_last - 1].n_series), int(ress[n_last - 1].n_candidates),
                                 int(ress[n_last - 1].n_decisions)))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_bits, last_counts)
 
     # ---- N > 1: where the step time goes (fused exchange only) ------------------------------------
     breakdown = None
@@ -655,7 +670,11 @@ def main():
                     help="c2 (default, the judged workload): 10k pods x 4 x 1800 per GPU, weak scaling.  "
                          "c4 / c5 (profiling only): BASELINE configs[3] / [4], a FIXED total of 250k x 4 x 1800 "
                          "/ 2.5M x 4 x 7200 pods sharded over the ranks (strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global PODS, GPUS, SAMPLES, ROTATE
     args.strong_total = 0
     if args.config != "c2":

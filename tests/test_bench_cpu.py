@@ -72,6 +72,32 @@ def test_config_is_identical_in_both_arms_and_reference_line_has_the_contract_ke
     assert abs(line["value"] - b.PODS * b.GPUS * b.SAMPLES / (line["ms_per_step"] * 1e-3)) / line["value"] < 1e-6
 
 
+def test_dump_outputs_hold_the_last_timed_step(bench, tmp_path, monkeypatch, capsys):
+    """--dump-outputs: the bitmap and counts of the LAST of the K timed steps (window (K - 1) % ROTATE), as float64"""
+    import argparse
+    from oracle import oracle_c
+    monkeypatch.setattr(oracle_c, "pool_pin", lambda on=True: None)   # keep this process's oracle pool unpinned
+    steps = 3
+    args = argparse.Namespace(gpus=1, steps=steps, warmup=3, dump_outputs=str(tmp_path / "out"))
+    assert bench.run_reference(args) == 0
+    line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
+    assert line["steps"] == steps
+    bits, counts = np.load(tmp_path / "out" / "decision_bits.npy"), np.load(tmp_path / "out" / "counts.npy")
+    assert bits.dtype == counts.dtype == np.float64
+    ref = oracle_c.decide_synth(bench.SEED + 16 * ((steps - 1) % bench.ROTATE), 0, bench.PODS, bench.GPUS, bench.SAMPLES,
+                                use_elig=True, n_threads=2)
+    assert np.array_equal(bits, ref["decision_bits"].astype(np.float64))
+    assert counts.tolist() == [ref["n_series"], ref["n_candidates"], ref["n_decisions"]]
+    other = oracle_c.decide_synth(bench.SEED, 0, bench.PODS, bench.GPUS, bench.SAMPLES, use_elig=True, n_threads=2)
+    assert not np.array_equal(other["decision_bits"], ref["decision_bits"])   # the window really tells the steps apart
+
+
+def test_steps_below_one_are_refused():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=300)
+    assert p.returncode == 2 and "--steps" in p.stderr
+
+
 def test_cuda_arm_refuses_to_run_without_a_gpu():
     import torch
     if torch.cuda.is_available():
